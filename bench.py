@@ -2,7 +2,7 @@
 """bench.py — image-pairs matched/sec on the descriptor-matching hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1|2|3|sweep]
-                    [--features M] [--images I] [--dtype f32|u8|bin] [--data int|real] [--cpu-seconds S]
+                    [--features M] [--images I] [--dtype f32|u8|bin] [--data int|real] [--cpu-seconds S] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the rank's shard of the pair list.  Default (N=1): BASELINE configs[1],
 100 synthetic images x 8192 SIFT features, exhaustive 4950 pairs.  Printed by rank 0 as ONE JSON line:
@@ -61,7 +61,11 @@ def parse():
     ap.add_argument("--sharding", default="2d", choices=["2d", "rows"], help="multi-rank split of the pair list: 2-D blocks (default) or by database image")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned to DIR/<name>.npy (float32 / float64, a seeded sample of the match lists)")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs dumps the GPU path (--impl ours)")
     if a.config == "3":
         a.dtype = "bin"
     a.features = a.features or (16384 if a.config == "3" else 8192)
@@ -274,6 +278,31 @@ def workload_text(args, n_img, n_pairs):
             f"BRUTE_FORCE_{'HAMMING' if hamming else 'L2'}, ratio 0.8")
 
 
+DUMP_SAMPLE_BYTES = 48 << 20     # the sampled match lists; the per-pair arrays add well under 1 MB at 4950 pairs
+
+
+def dump_outputs(out_dir, pair_ids, offsets, matches, max_features):
+    """What the timed path returned (pair ids, CSR offsets, match records i / j / ratio / dist) as DIR/<name>.npy in float64 /
+    float32: the pair list and offsets, per-pair sums of ratio and dist over every match, and the complete match lists of a
+    seeded sample of pairs.  The sample depends on the inputs only (pair count, features per view: at most one match per query
+    feature), so two builds dump the same pairs, and it is sized to keep the files under 64 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(pair_ids)
+    counts = np.diff(offsets)
+    owner = np.repeat(np.arange(n), counts)
+    k = min(n, max(1, DUMP_SAMPLE_BYTES // (24 * max(1, max_features))))
+    sample = np.sort(np.random.default_rng(0).permutation(n)[:k])
+    rows = np.concatenate([np.arange(offsets[p], offsets[p + 1]) for p in sample]) if k else np.zeros(0, np.int64)
+    arrays = {"pair_ids": pair_ids.astype(np.float64), "offsets": offsets.astype(np.float64),
+              "ratio_sum_per_pair": np.bincount(owner, weights=matches["ratio"], minlength=n),
+              "dist_sum_per_pair": np.bincount(owner, weights=matches["dist"], minlength=n),
+              "sample_pair_index": sample.astype(np.float64), "sample_offsets": np.concatenate([[0], np.cumsum(counts[sample])]).astype(np.float64),
+              "sample_i": matches["i"][rows].astype(np.float64), "sample_j": matches["j"][rows].astype(np.float64),
+              "sample_ratio": matches["ratio"][rows], "sample_dist": matches["dist"][rows]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
+
+
 def pin_to_gpu_numa_node(local: int) -> str:
     """One rank per GPU on a two-socket host: keep this process (its pinned buffers, the engine's threads) on the GPU's NUMA node."""
     try:
@@ -391,13 +420,19 @@ def main():
     barrier()
     t0w = time.time()
     gpu_ms = 0.0; search_ms = 0.0; launches = 0; records = 0
+    last = None
     for _ in range(args.steps):
-        m.match_uploaded(mine, matching.STAGE_FULL)
+        last = None                                   # a step's result is freed before the next step runs
+        last = m.match_uploaded(mine, matching.STAGE_FULL)
         gpu_ms += ctx.last_gpu_ms(); search_ms += ctx.last_search_kernel_ms(); launches += ctx.last_launches(); records += ctx.last_records()
     barrier()
     t1w = time.time()
     clocks = sampler.stop(t0w, t1w) if sampler else None
     tc_pairs = ctx.last_tc_pairs(); errs = ctx.exactness_errors(); real_pairs = ctx.last_real_tc_pairs(); fb_rows = ctx.last_fallback_rows()
+    if args.dump_outputs and last is not None:
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"), *last,
+                     max((len(d) for d, _ in my_views.values()), default=1))
+    last = None
 
     # ---- e2e: host buffers -> upload -> match -> D2H -> finishing -> result arrays -------------------------------------
     e2e_s = 0.0; h2d = 0; d2h = 0; e2e_steps = 0

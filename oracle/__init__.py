@@ -13,6 +13,7 @@ legs may import this package.  The product (alicevision_b200/) never does.
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import os
 import subprocess
 
@@ -20,6 +21,8 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 DT_F32, DT_U8, DT_BIN = 0, 1, 2
+# outputs of the compiled reference on the inputs of the port-equals-reference tests (tests/golden/make_golden.py parity)
+PARITY = os.path.join(os.path.dirname(_HERE), "tests", "golden", "reference_parity.npz")
 
 MATCH_DTYPE = np.dtype([("i", np.uint32), ("j", np.uint32), ("ratio", np.float32), ("dist", np.float32)])
 
@@ -309,6 +312,25 @@ class VoctreeOracle:
                                                            C.c_long(numImageQuery), _p(mids), _p(sc), _p(w), _p(pairs), C.c_long(cap), C.byref(npairs))
         assert r == keep, (r, keep)
         return ids, mids[:, :keep], sc[:, :keep], w, pairs[: npairs.value].copy()
+
+
+def stored_reference(prefix: str) -> dict:
+    """The compiled reference's outputs stored under `prefix` in tests/golden/reference_parity.npz, by name."""
+    with np.load(PARITY) as g:
+        return {k.split("__", 1)[1]: g[k] for k in g.files if k.startswith(prefix + "__")}
+
+
+def assert_outputs_equal(got: dict, want: dict, who: str) -> None:
+    """Every named output of `got` equals the stored one, bit for bit (structured match records included)."""
+    assert sorted(got) == sorted(want), (who, sorted(set(got) ^ set(want)))
+    for k in want:
+        assert np.asarray(got[k]).dtype == want[k].dtype and np.array_equal(got[k], want[k]), f"{who}: {k} differs from the reference's stored output"
+
+
+def sha256(data) -> np.ndarray:
+    """SHA-256 of a file (path) or of an array's bytes, as 32 uint8: how the tests store large reference outputs compared byte for byte."""
+    raw = open(data, "rb").read() if isinstance(data, str) else np.ascontiguousarray(data).tobytes()
+    return np.frombuffer(hashlib.sha256(raw).digest(), np.uint8)
 
 
 def best(prefer_ref: bool = True) -> Oracle:

@@ -1,7 +1,8 @@
 """Generates tests/golden/*.npz from the REFERENCE itself (oracle/_ref/libref_oracle.so = the reference's own
-headers compiled verbatim from /root/reference/src).  Run in the build container:  python tests/golden/make_golden.py
-The fixtures pin both the port oracle (CPU tests) and the CUDA path (GPU tests) to reference outputs even where
-/root/reference is absent."""
+headers compiled verbatim from the reference tree, oracle/Makefile REF).  Where the reference tree is present:
+    python tests/golden/make_golden.py [io | parity]
+The fixtures pin both the port oracle (CPU tests) and the CUDA path (GPU tests) to reference outputs where the compiled
+reference is absent."""
 import os
 import sys
 
@@ -79,9 +80,39 @@ def io_golden():
     print("wrote io_golden.npz and io_{u8,f32,bin}.{feat,desc}")
 
 
+def parity():
+    """reference_parity.npz: what the port-equals-reference tests compare, computed by the compiled reference (the tests' own
+    functions, so inputs and outputs cannot drift apart).  Large byte-for-byte outputs are stored as SHA-256 digests."""
+    import tempfile
+    oracle.build(ref=True)
+    sys.path.insert(0, os.path.dirname(HERE))
+    import test_guided, test_io, test_oracle, test_voctree  # noqa: E401
+    out = {}
+
+    def put(prefix, outputs):
+        out.update({f"{prefix}__{k}": np.asarray(v) for k, v in outputs.items()})
+
+    R = oracle.Oracle("ref")
+    put("oracle", test_oracle.port_reference_outputs(R))
+    for kind in ("u8", "f32", "real", "bin"):
+        put(f"guided_{kind}", test_guided.reference_outputs(R, kind))
+    put("guided_homography", test_guided.homography_reference_outputs(R))
+    with tempfile.TemporaryDirectory() as t:
+        for method in test_voctree.METHODS:
+            put(f"voctree_{method}", test_voctree.reference_outputs(oracle.VoctreeOracle("ref"), method, t))
+        for what in ("u8", "f32", "bin"):
+            put(f"io_{what}", test_io.reference_regions_outputs(R, what, t))
+        put("io_conversion", test_io.reference_conversion_outputs(R, t))
+    np.savez_compressed(oracle.PARITY, **out)
+    print(f"wrote {oracle.PARITY}: {len(out)} arrays")
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "io":
         io_golden()
+    elif len(sys.argv) > 1 and sys.argv[1] == "parity":
+        parity()
     else:
         main()
         io_golden()
+        parity()

@@ -87,3 +87,32 @@ def test_reference_arm_runs_on_the_cpu():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"], capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_dump_outputs(tmp_path):
+    """--dump-outputs: float32 / float64 arrays only; the sampled match lists are the returned records of the sampled pairs, the
+    per-pair sums cover every record, and the sample is the same on every run."""
+    import numpy as np
+    import bench
+    from alicevision_b200 import synth
+    from alicevision_b200.matching import MATCH_DTYPE
+    rng = np.random.default_rng(1)
+    pairs = synth.exhaustive_pairs(40)
+    offsets = np.concatenate([[0], np.cumsum(rng.integers(0, 30, len(pairs)))]).astype(np.int64)
+    m = np.zeros(int(offsets[-1]), MATCH_DTYPE)
+    m["i"] = rng.integers(0, 1 << 32, len(m)); m["j"] = rng.integers(0, 1 << 32, len(m)); m["ratio"] = rng.random(len(m)); m["dist"] = rng.random(len(m)) * 1e5
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), pairs, offsets, m, max_features=200000)
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    assert all(np.array_equal(a, np.load(tmp_path / "b" / f"{k}.npy")) for k, a in got.items())
+    assert np.array_equal(got["pair_ids"], pairs) and np.array_equal(got["offsets"], offsets)
+    sums = [m["dist"][a:b].astype(np.float64).sum() for a, b in zip(offsets[:-1], offsets[1:])]
+    assert np.allclose(got["dist_sum_per_pair"], sums, rtol=1e-12)
+    sample = got["sample_pair_index"].astype(np.int64)
+    assert 0 < len(sample) < len(pairs) and np.all(np.diff(sample) > 0)      # 48 MB / (24 B x 200000 features): 10 pairs
+    so = got["sample_offsets"].astype(np.int64)
+    for k, p in enumerate(sample):
+        want = m[offsets[p]:offsets[p + 1]]
+        assert np.array_equal(got["sample_i"][so[k]:so[k + 1]], want["i"]) and np.array_equal(got["sample_j"][so[k]:so[k + 1]], want["j"])
+        assert np.array_equal(got["sample_ratio"][so[k]:so[k + 1]], want["ratio"]) and np.array_equal(got["sample_dist"][so[k]:so[k + 1]], want["dist"])

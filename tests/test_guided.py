@@ -73,17 +73,39 @@ def kinds():
     return [k for k in ("ref", "port") if oracle.available(k)]
 
 
-@pytest.mark.skipif(len(kinds()) < 2, reason="needs both the compiled reference and the port")
+def reference_outputs(o, kind):
+    """test_port_equals_reference's guided matches for one descriptor type, computed by oracle `o` (make_golden.py stores the
+    compiled reference's)."""
+    Fg, A = general_F()
+    out = {}
+    for f, (F, AA) in enumerate(((F_RECT, None), (Fg, A))):
+        dl, xl, dr, xr, _ = scene(kind, 700, A=AA)
+        for th, ratio in ((4.0, 0.64), (16.0, 0.36), (0.25, 0.9)):
+            out[f"F{f}_{th:g}_{ratio:g}"] = o.guided_match(dl, xl, dr, xr, F, th, ratio, binary=kind == "bin")
+    return out
+
+
+def homography_reference_outputs(o):
+    """test_port_equals_reference_homography's guided matches, computed by oracle `o`."""
+    out = {}
+    for kind in ("u8", "real", "bin"):
+        dl, xl, dr, xr, _, H = homography_scene(kind, 600)
+        for th, ratio in ((400.0, 0.64), (900.0, 0.36)):
+            out[f"{kind}_{th:g}_{ratio:g}"] = o.guided_match(dl, xl, dr, xr, H, th, ratio, binary=kind == "bin", model=1)
+    return out
+
+
 @pytest.mark.parametrize("kind", ["u8", "f32", "real", "bin"])
 def test_port_equals_reference(kind):
-    R, P = oracle.Oracle("ref"), oracle.Oracle("port")
-    Fg, A = general_F()
-    for F, AA in ((F_RECT, None), (Fg, A)):
-        dl, xl, dr, xr, truth = scene(kind, 700, A=AA)
-        for th, ratio in ((4.0, 0.64), (16.0, 0.36), (0.25, 0.9)):
-            a = R.guided_match(dl, xl, dr, xr, F, th, ratio, binary=kind == "bin"); b = P.guided_match(dl, xl, dr, xr, F, th, ratio, binary=kind == "bin")
-            assert np.array_equal(a, b)
-        a = R.guided_match(dl, xl, dr, xr, F, 4.0, 0.64, binary=kind == "bin")
+    """The restated guided matching equals the reference's; its outputs are stored (tests/golden/make_golden.py) and recomputed
+    where the compiled reference is present."""
+    want = oracle.stored_reference(f"guided_{kind}")
+    for k in kinds():
+        oracle.assert_outputs_equal(reference_outputs(oracle.Oracle(k), kind), want, k)
+    _, A = general_F()
+    for f, AA in enumerate((None, A)):
+        truth = scene(kind, 700, A=AA)[4]
+        a = want[f"F{f}_4_0.64"]
         good = sum(1 for m in a if truth.get(int(m["i"])) == int(m["j"]))
         assert len(a) > 100 and good > 0.9 * len(a)
 
@@ -105,15 +127,13 @@ def test_gpu_guided_matching_equals_oracle(kind):
         assert len(matching.guidedMatching(F, L, Rr, 4.0, 0.64)) > 300
 
 
-@pytest.mark.skipif(len(kinds()) < 2, reason="needs both the compiled reference and the port")
 def test_port_equals_reference_homography():
-    R, P = oracle.Oracle("ref"), oracle.Oracle("port")
+    want = oracle.stored_reference("guided_homography")
+    for k in kinds():
+        oracle.assert_outputs_equal(homography_reference_outputs(oracle.Oracle(k)), want, k)
     for kind in ("u8", "real", "bin"):
-        dl, xl, dr, xr, truth, H = homography_scene(kind, 600)
-        for th, ratio in ((400.0, 0.64), (900.0, 0.36)):
-            a = R.guided_match(dl, xl, dr, xr, H, th, ratio, binary=kind == "bin", model=1); b = P.guided_match(dl, xl, dr, xr, H, th, ratio, binary=kind == "bin", model=1)
-            assert np.array_equal(a, b)
-        a = R.guided_match(dl, xl, dr, xr, H, 400.0, 0.64, binary=kind == "bin", model=1)
+        truth = homography_scene(kind, 600)[4]
+        a = want[f"{kind}_400_0.64"]
         assert len(a) > 100 and sum(1 for m in a if truth.get(int(m["i"])) == int(m["j"])) > 0.9 * len(a)
 
 

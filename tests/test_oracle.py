@@ -75,33 +75,46 @@ def test_ratio_filter_semantics(oracles, kind):
     assert keep.tolist() == [0, 2] and ratios.tolist() == [0.0, 0.0]      # integer division -> 0
 
 
-@pytest.mark.skipif(not (oracle.available("ref") or os.path.isdir("/root/reference/src")), reason="compiled reference not available")
-def test_port_equals_reference(oracles):
-    """The restatement must equal the reference's own headers on every stage, including tie order and the
-    non-strict-weak-order coordinate de-duplication (adversarial positions)."""
-    R, P = oracles["ref"], oracles["port"]
+def _packed(prefix, res):
+    """{(I, J): matches} as three arrays: sorted pairs, offsets, concatenated matches."""
+    keys = sorted(res)
+    return {f"{prefix}_pairs": np.array(keys, np.uint32).reshape(-1, 2), f"{prefix}_off": np.cumsum([0] + [len(res[k]) for k in keys]).astype(np.int64),
+            f"{prefix}_matches": np.concatenate([res[k] for k in keys]) if keys else np.zeros(0, oracle.MATCH_DTYPE)}
+
+
+def port_reference_outputs(o):
+    """Every stage test_port_equals_reference compares, computed by oracle `o` (make_golden.py stores the compiled reference's)."""
+    out = {}
     rng = np.random.default_rng(0)
     descs, xys = synth.sift_images(3, 400, np.uint8, seed=3, pool_factor=1.0)
-    for ds in (descs, [d.astype(np.float32) for d in descs], synth.real_valued(descs)):
-        okr, ir, dr = R.knn(ds[0], ds[1], 2); okp, ip, dp = P.knn(ds[0], ds[1], 2)
-        assert okr and okp and np.array_equal(ir, ip) and np.array_equal(dr, dp)
+    pairs = synth.exhaustive_pairs(3)
+    for name, ds in (("u8", descs), ("f32", [d.astype(np.float32) for d in descs]), ("real", synth.real_valued(descs))):
+        ok, out[f"knn_{name}_idx"], out[f"knn_{name}_dist"] = o.knn(ds[0], ds[1], 2)
+        assert ok
         for cross in (False, True):
-            a, b = R.collection_match(ds, xys, synth.exhaustive_pairs(3), 0.8, cross), P.collection_match(ds, xys, synth.exhaustive_pairs(3), 0.8, cross)
-            assert a.keys() == b.keys() and all(np.array_equal(a[k], b[k]) for k in a)
+            out.update(_packed(f"{name}_cross{int(cross)}", o.collection_match(ds, xys, pairs, 0.8, cross)))
     # heavy ties: tiny alphabet
     t = rng.integers(0, 2, (200, 128)).astype(np.uint8)
-    okr, ir, dr = R.knn(t[:100], t[100:], 2); okp, ip, dp = P.knn(t[:100], t[100:], 2)
-    assert np.array_equal(dr, dp) and np.array_equal(ir, ip)
+    _, out["ties_idx"], out["ties_dist"] = o.knn(t[:100], t[100:], 2)
     # adversarial positions
     _, axy = synth.sift_images(3, 400, np.uint8, seed=3, pool_factor=1.0, generic_positions=False)
-    a, b = R.collection_match(descs, axy, synth.exhaustive_pairs(3), 0.8), P.collection_match(descs, axy, synth.exhaustive_pairs(3), 0.8)
-    assert a.keys() == b.keys() and all(np.array_equal(a[k], b[k]) for k in a)
+    out.update(_packed("adv", o.collection_match(descs, axy, pairs, 0.8)))
     m = np.zeros(300, oracle.MATCH_DTYPE); m["i"] = rng.integers(0, 50, 300); m["j"] = rng.integers(0, 400, 300)
-    m = R.indmatch_dedup(m)
-    assert np.array_equal(R.decorator_dedup(m, axy[0], axy[1]), P.decorator_dedup(m, axy[0], axy[1]))
+    out["indmatch_dedup"] = m = o.indmatch_dedup(m)
+    out["decorator_dedup"] = o.decorator_dedup(m, axy[0], axy[1])
     bd, bxy = synth.mldb_images(2, 300)
-    a, b = R.regions_match(bd[0], bxy[0], bd[1], bxy[1], 0.8, True), P.regions_match(bd[0], bxy[0], bd[1], bxy[1], 0.8, True)
-    assert a[0] == b[0] and np.array_equal(a[1], b[1])
+    ok, out["bin_regions_match"] = o.regions_match(bd[0], bxy[0], bd[1], bxy[1], 0.8, True)
+    out["bin_regions_ok"] = np.array(ok)
+    return out
+
+
+def test_port_equals_reference(oracles):
+    """The restatement must equal the reference's own headers on every stage, including tie order and the
+    non-strict-weak-order coordinate de-duplication (adversarial positions).  The compiled reference's outputs are stored
+    (tests/golden/make_golden.py); where the compiled reference is present it must still produce them."""
+    want = oracle.stored_reference("oracle")
+    for kind, o in oracles.items():
+        oracle.assert_outputs_equal(port_reference_outputs(o), want, kind)
 
 
 @pytest.mark.parametrize("kind", kinds())

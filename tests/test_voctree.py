@@ -33,19 +33,34 @@ def tree(seed=4, invalid_tail=1):
     return synth.vocabulary_tree(K, L, seed=seed, invalid_tail=invalid_tail)
 
 
-@pytest.mark.skipif(len(kinds()) < 2, reason="needs both the compiled reference and the port")
-@pytest.mark.parametrize("method", ["strongCommonPoints", "commonPoints", "classic", "inversedWeightedCommonPoints"])
-def test_port_equals_reference(method, tmp_path):
-    R, P = oracle.VoctreeOracle("ref"), oracle.VoctreeOracle("port")
+METHODS = ["strongCommonPoints", "commonPoints", "classic", "inversedWeightedCommonPoints"]
+
+
+def reference_outputs(o, method, tmp_dir):
+    """Words, then (query ids, ranked matches, scores, weights, pair list) for three query settings, computed by voctree oracle `o`
+    (make_golden.py stores the compiled reference's)."""
     c, v = tree()
     d = views()
-    for descs in (d[3], d[5].astype(np.float32), synth.real_valued([d[8 if len(d[8]) else 13]])[0]):
-        assert np.array_equal(R.quantize(K, L, c, v, descs, str(tmp_path / "t.tree")), P.quantize(K, L, c, v, descs))
+    tree_path = os.path.join(tmp_dir, "t.tree")
+    out = {}
+    for n, descs in enumerate((d[3], d[5].astype(np.float32), synth.real_valued([d[8 if len(d[8]) else 13]])[0])):
+        out[f"words{n}"] = o.quantize(K, L, c, v, descs, tree_path)
     for nq, nmax in ((0, 0), (4, 0), (3, 200)):
-        a = R.image_matching(K, L, c, v, d, nmax, nq, method, str(tmp_path / "t.tree")); b = P.image_matching(K, L, c, v, d, nmax, nq, method)
-        for x, y in zip(a, b):
-            assert np.array_equal(x, y)
-        assert len(a[4]) > 0 and np.all(a[4][:, 0] != a[4][:, 1])
+        for name, x in zip(("ids", "matches", "scores", "weights", "pairs"), o.image_matching(K, L, c, v, d, nmax, nq, method, tree_path)):
+            out[f"{name}_q{nq}_max{nmax}"] = x
+    return out
+
+
+@pytest.mark.parametrize("method", METHODS)
+def test_port_equals_reference(method, tmp_path):
+    """The restatement equals the reference's own voctree code; its outputs are stored (tests/golden/make_golden.py) and
+    recomputed where the compiled reference is present."""
+    want = oracle.stored_reference(f"voctree_{method}")
+    for k in kinds():
+        oracle.assert_outputs_equal(reference_outputs(oracle.VoctreeOracle(k), method, str(tmp_path)), want, k)
+    for nq, nmax in ((0, 0), (4, 0), (3, 200)):
+        p = want[f"pairs_q{nq}_max{nmax}"]
+        assert len(p) > 0 and np.all(p[:, 0] != p[:, 1])
 
 
 def test_words_spread_over_the_vocabulary():
